@@ -3,7 +3,7 @@
 (BASELINE.json configs[1], "C2").  One "step" = one pass of the hot path (boundary tensors ->
 ingest -> solve -> adjoint -> emit) over one batch of synthetic dense QPs.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch B]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch B] [--dump-outputs DIR]
 
 * ours      : `value` = device-resident throughput (inputs already in HBM), `e2e` = the same step
               through the reference-facing `_CvxpyLayer.apply` with HOST buffers (H2D + D2H inside
@@ -143,6 +143,31 @@ def config_block(bt, B: int, world: int, l2: str) -> dict:
 def l2_note(st, B: int) -> str:
     nbytes = (st.nnzA + st.m + st.n + 1 + st.nnzP) * B * 8
     return f"inputs ({nbytes / 1e9:.2f} GB/step) vs 126 MB L2" + ("" if nbytes > 130e6 else "; NOT larger than L2 (secondary config, no flush)")
+
+
+DUMP_BYTES = 60 * 10**6   # --dump-outputs budget (under 64 MB with the .npy headers); beyond it a seeded sample of instances
+
+
+def dump_outputs(out_dir: str, sol, grads, B: int):
+    """Writes what one step of the timed path hands its caller -- the solution (x, y, s, status) and the gradients of the
+    boundary tensors (A_eval, q_eval, P_eval) -- as float64 .npy files, for the instances listed in `instances.npy`: all of
+    them when that fits DUMP_BYTES, else a sorted sample drawn with a fixed seed, so two builds dump the same instances."""
+    import torch
+
+    gA, gq, gP = grads
+    per_instance = 8 * (sol.x.shape[1] + sol.y.shape[1] + sol.s.shape[1] + 2 + gA.shape[0] + gq.shape[0] + (gP.shape[0] if gP is not None else 0))
+    k = min(B, DUMP_BYTES // per_instance)
+    idx = np.arange(B) if k == B else np.sort(np.random.default_rng(0).choice(B, size=k, replace=False))
+    it = torch.as_tensor(idx, device=sol.x.device)
+    arrays = {"instances": idx, "x": sol.x[it], "y": sol.y[it], "s": sol.s[it], "status": sol.status[it],
+              "grad_A_eval": gA[:, it], "grad_q_eval": gq[:, it]}
+    if gP is not None:
+        arrays["grad_P_eval"] = gP[:, it]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, v in arrays.items():
+        v = v.cpu().numpy() if isinstance(v, torch.Tensor) else v
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.ascontiguousarray(v, dtype=np.float64))
+    print(f"[bench] outputs of the last timed step ({k} of {B} instances) written to {out_dir}", file=sys.stderr)
 
 
 def host_cores() -> int:
@@ -483,6 +508,8 @@ def run_ours(a):
     sync()
     if world == 1:
         clocks = sampler.stop()
+        if a.dump_outputs:
+            dump_outputs(a.dump_outputs, sol, dbuf["ev"], B)
     launches = eng.launch_count() - l0
     ms_total = t_start.elapsed_time(t_end)
     for e in evs:
@@ -510,6 +537,8 @@ def run_ours(a):
             return float(tt), sol_, its_, eng.launch_count() - lA
         ms_step, sol, its, launches = timed_sharded(B, a.chunk)  # weak scaling: every rank its own B instances
         clocks = sampler.stop()
+        if a.dump_outputs and rank == 0:   # rank 0's own shard
+            dump_outputs(a.dump_outputs, sol, (bufs["gA_eval"], bufs["gq_eval"], bufs["gP_eval"]), B)
         Bs = max(1, B // world)                                  # strong scaling: the BASELINE batch split over the ranks
         ms_strong, _, _, _ = timed_sharded(Bs, a.chunk)
         strong = {"global_batch": Bs * world, "batch_per_gpu": Bs, "ms_per_step": ms_strong, "value": Bs * world / (ms_strong * 1e-3), "unit": UNIT,
@@ -543,7 +572,7 @@ def run_ours(a):
         loss_val, gAh, gqh, gPh = step_e2e()
     sync()
     e0, e1 = ev(), ev()
-    n_e2e = max(1, a.steps)
+    n_e2e = a.steps
     per_step = []
     e0.record()
     for _ in range(n_e2e):
@@ -568,17 +597,17 @@ def run_ours(a):
             step_e2e(True)
         sync()
         tw = time.perf_counter()
-        for _ in range(3):
+        for _ in range(a.steps):
             step_e2e(True)
         sync()
-        e2e_pageable = {"value": Btot / ((time.perf_counter() - tw) / 3), "unit": UNIT, "steps": 3,
+        e2e_pageable = {"value": Btot / ((time.perf_counter() - tw) / a.steps), "unit": UNIT, "steps": a.steps,
                         "note": "pageable host inputs (the reference's CPU tensors): batch slices gathered into a ring of pinned staging buffers by a background thread, then the same two-stream pipeline"}
         del pA, pq, pP
     # f1 + f2 in one number: only parameters cross PCIe, the matrices are constants of the layer
     e2e_fused = None
     if world == 1 and CONFIG == "C2" and rank == 0:
         try:
-            e2e_fused = fused_param_variant(bt, B, dev, SOLVER_ARGS, max(3, min(a.steps, 10)), a.warmup)
+            e2e_fused = fused_param_variant(bt, B, dev, SOLVER_ARGS, a.steps, a.warmup)
         except Exception as ex:  # noqa: BLE001  (a secondary measurement must not take the line down)
             e2e_fused = {"error": repr(ex)[:300]}
     npel = hP.numel() if hP is not None else 0
@@ -654,7 +683,11 @@ def main():
     p.add_argument("--verify-exchange", action="store_true", help="N > 1: check rank 0's gathered buffer against an NCCL gather")
     p.add_argument("--set", action="append", default=[], metavar="KEY=VALUE",
                    help="override a solver argument for both arms, e.g. --set acceleration_lookback=0")
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="write the solution and gradients of the last timed step as DIR/<name>.npy (float64, at most 64 MB)")
     a = p.parse_args()
+    if a.steps < 1:
+        p.error("--steps must be at least 1")
     a.cpu_sample_given = a.cpu_sample is not None
     if a.cpu_sample is None:
         a.cpu_sample = 2048

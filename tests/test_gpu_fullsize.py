@@ -3,8 +3,8 @@
 * every BASELINE config at its real batch (C2 4096, C3 2048, C4 512 forward AND backward at n=1000/m=2000, C5 256):
   work-queue, wave and multi-CTA/SM effects are only exercised there;
 * the gradient a user actually gets -- GPU adjoint at the GPU's OWN solution -- against the oracle's pipeline;
-* the reference's own finite-difference programs (PSD: /root/reference/tests/test_torch.py:233-248, SOC:
-  /root/reference/tests/test_dual_variables.py:346-369, atol 1e-4 / rtol 1e-3) through the CUDA path;
+* the reference's own finite-difference programs (PSD: cvxpylayers tests/test_torch.py:233-248, SOC:
+  cvxpylayers tests/test_dual_variables.py:346-369, atol 1e-4 / rtol 1e-3) through the CUDA path;
 * every LSQR variant against an EXACT dense least-squares solve of diffcp's adjoint system, which is what justifies the
   tolerance of the reference-semantics recurrence (lsqr_precond = 0).
 

@@ -28,7 +28,7 @@ def rel_err(a, b):
 # ----------------------------------------------------------------------------- the reference's own gradcheck programs
 def ref_sdp_batch(C_list):
     """``min tr(C X) s.t. tr(X) = 1, X >> 0`` for 3 x 3 symmetric C -- the program of the reference's PSD
-    gradcheck (``/root/reference/tests/test_torch.py:233-248``) written directly in solver form with x = svec(X)
+    gradcheck (cvxpylayers ``tests/test_torch.py:233-248``) written directly in solver form with x = svec(X)
     (lower triangle, column-major, off-diagonals * sqrt 2): one zero-cone row for the trace, -x + s = 0 with s in the
     PSD cone.  The optimum is the rank-one projector on the smallest eigenvector of C and is strictly complementary
     when that eigenvalue is simple, so the solution map is differentiable.  One instance per C in ``C_list``."""
@@ -48,7 +48,7 @@ def ref_sdp_batch(C_list):
 
 def ref_soc_batch(c_list, t_list):
     """``min c'x + 0.1 ||x||^2 s.t. ||x|| <= t`` (n = 3) -- the program of the reference's SOC gradcheck
-    (``/root/reference/tests/test_dual_variables.py:346-369``) in solver form: P = 0.2 I, one SOC of size 4 with
+    (cvxpylayers ``tests/test_dual_variables.py:346-369``) in solver form: P = 0.2 I, one SOC of size 4 with
     s = (t, x).  Outputs of the reference's check: the SOC dual (sum), parameters c and t."""
     n = 3
     indptr = [0, 0, 1, 2, 3]
@@ -66,7 +66,7 @@ def install_fake_cvxpylayers(monkeypatch):
     layout in ``sys.modules`` to drive ``cvxpylayers_b200.interface.register()`` the way the real package would:
 
     * ``cvxpylayers.interfaces.get_solver_ctx / get_torch_cvxpylayer`` -- closed dispatch that rejects unknown names
-      (``/root/reference/src/cvxpylayers/interfaces/__init__.py:13-101``);
+      (cvxpylayers ``src/cvxpylayers/interfaces/__init__.py:13-101``);
     * ``cvxpylayers.utils.parse_args.parse_args(problem, variables, parameters, solver, ...)`` -- refuses solver names
       cvxpy does not know (that is what ``problem.get_problem_data(solver=...)`` does, ``parse_args.py:447-462``), then
       calls ``interfaces.get_solver_ctx`` and returns a LayersContext-like dataclass;
